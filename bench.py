@@ -2,7 +2,7 @@
 """Benchmark of the SM3Det sparse-MoE backbone hot path (BASELINE.json metric: backbone images/s @1024^2, bs = 32).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                  [--config t_e8|b_e16|lsk_s] [--global-batch G | --batch B] [--expert-parallel]
+                  [--config t_e8|b_e16|lsk_s] [--global-batch G | --batch B] [--expert-parallel] [--dump-outputs DIR]
 
 One "step" = forward + backward of the backbone over the GLOBAL batch of synthetic 1024^2 tiles:
   t_e8  (default) BASELINE configs[1]/[2]: ConvNeXt-T, E = 8 top-2, MoE in the last two stages every other block.
@@ -81,7 +81,15 @@ def parse():
                          'auto = flat when the step is graph-captured')
     ap.add_argument('--no-grad-sync', action='store_true',
                     help='DIAGNOSTIC, N > 1: never all-reduce gradients (isolates the exposed cost of the DDP collective)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last step returned (rank 0: feature maps, gate losses, step loss, '
+                         'parameter gradients) as DIR/<name>.npy; inputs, weights and gating noise are seeded, so two builds '
+                         'run with the same arguments can be compared file by file')
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and a.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of --impl ours')
     for c in CONFIGS.values():            # applies to both arms (ours and --impl reference) and to the oracle baselines
         if c['family'] == 'convnext':
             c['kw']['noisy_gating'] = a.noisy_gating == 'config'
@@ -214,7 +222,7 @@ def run_reference(args):
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
         return
-    steps, warmup = max(1, min(args.steps, 3)), min(args.warmup, 1)
+    steps, warmup = args.steps, args.warmup
     ips, dt, threads, fwd_ips = time_cpu_reference(args, args.cpu_images, steps, warmup)
     _, _, _, scaling, _ = resolve(args, args.gpus)
     line = {'impl': 'reference', 'metric': METRIC, 'value': ips, 'unit': 'img/s', 'n_gpus': args.gpus, 'steps': steps,
@@ -376,6 +384,43 @@ def moe_roofline(net, x, peaks):
     return out
 
 
+DUMP_FEATURE_SAMPLES = 1 << 20     # elements kept of each feature level (float32: 4 MB)
+DUMP_GRAD_SAMPLES = 1 << 23        # elements kept of all parameter gradients together (32 MB)
+
+
+def dump_outputs(path, kept):
+    """--dump-outputs: the last step's results as .npy files, 48 MB and a few kB at most.  Tensors above their budget are
+    reduced to a fixed-seed sample of elements (same shapes -> same positions), plus the float64 L2 norm of every full tensor:
+      features_<i>   level i of the backbone output over the per-GPU batch (micro-batches concatenated), float32
+      feature_l2     L2 norm of each full level, float64
+      gate_loss      load-balance loss of each micro-batch, float32
+      step_loss      the value the step returns (sum of the levels' means + gate loss, over the micro-batches), float32
+      grads          samples of every parameter gradient, in named_parameters() order, concatenated, float32
+      grad_l2        L2 norm of each full parameter gradient, float64"""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+
+    def sample(t, n, seed):
+        t = t.detach().reshape(-1)
+        if t.numel() > n:
+            idx = torch.randint(0, t.numel(), (n,), generator=torch.Generator().manual_seed(seed)).sort().values
+            t = t[idx.to(t.device)]
+        return t.float().cpu().numpy()
+
+    def l2(ts):
+        return np.array([torch.linalg.vector_norm(t.detach(), dtype=torch.float64).item() for t in ts])
+
+    levels = [torch.cat(per_micro) for per_micro in zip(*kept['outs'])]
+    grads = [g for g in kept['grads'] if g is not None]
+    per_grad = max(1, DUMP_GRAD_SAMPLES // len(grads))
+    files = {f'features_{i}': sample(f, DUMP_FEATURE_SAMPLES, i) for i, f in enumerate(levels)}
+    files.update(feature_l2=l2(levels), gate_loss=torch.stack(kept['gate_loss']).float().cpu().numpy(),
+                 step_loss=kept['loss'].float().cpu().numpy(),
+                 grads=np.concatenate([sample(g, per_grad, 1000 + j) for j, g in enumerate(grads)]), grad_l2=l2(grads))
+    for name, a in files.items():
+        np.save(os.path.join(path, name + '.npy'), a)
+
+
 def build_model(args, world, ep, ddp=True):
     import torch.distributed as dist
     from sm3det_b200.synth import make_state_dict
@@ -416,6 +461,9 @@ def run_ours(args):
     rank = int(os.environ.get('RANK', '0'))
     local = int(os.environ.get('LOCAL_RANK', '0'))
     torch.cuda.set_device(local)
+    # the gating noise and LSKNet's dropout seeds come from torch's default generators; unseeded, CUDA's starts from a
+    # different seed in every process, so repeated runs would not compute the same step
+    torch.manual_seed(rank)
     if world > 1:
         dist.init_process_group('nccl')
     lib = _lib.load()
@@ -435,10 +483,16 @@ def run_ours(args):
     n_micro = B // MB
     host_x = make_images(B, S, S, seed=1234 + rank).pin_memory()
     dev_x = host_x.cuda()
+    # --dump-outputs: references to what the latest step returned.  Under graph capture these are the graph's static
+    # tensors, which every replay rewrites.
+    kept = {}
 
     def micro_step(x):
         with torch.autocast('cuda', dtype=torch.bfloat16, enabled=args.amp):
             outs, loss = model(x)
+        if args.dump_outputs:
+            kept['outs'].append([o.detach() for o in outs])
+            kept['gate_loss'].append(loss.detach())
         tot = (sum(o.float().mean() for o in outs) + loss) / n_micro
         tot.backward()
         return tot.detach()
@@ -446,6 +500,8 @@ def run_ours(args):
     def step(x):
         """one optimizer step's worth of work: fwd+bwd over the per-GPU batch, gradients accumulated over the micro-batches,
         all-reduced (DDP) once, during the last micro-batch's backward"""
+        if args.dump_outputs:
+            kept.update(outs=[], gate_loss=[])
         tot = None
         for i in range(n_micro):
             sync_ctx = model.no_sync() if (world > 1 and not flat_sync and (i + 1 < n_micro or args.no_grad_sync)) else contextlib.nullcontext()
@@ -454,6 +510,8 @@ def run_ours(args):
             tot = t if tot is None else tot + t
         if flat_sync and not args.no_grad_sync:
             allreduce_gradients(None, named=named_params, skip=ignored)
+        if args.dump_outputs:
+            kept.update(loss=tot, grads=[p.grad for _, p in named_params])
         return tot
 
     def sync():
@@ -556,6 +614,9 @@ def run_ours(args):
     if graphed is not None:       # the last replay's gradients are still in .grad: a checksum to cross-check micro-batch splits
         grad_l1 = float(sum(p.grad.double().abs().sum() for p in net.parameters() if p.grad is not None))
     peak_mem = torch.cuda.max_memory_allocated() / 2 ** 30
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, kept)     # before the instrumented passes below accumulate into .grad
+    kept.clear()
     t = torch.tensor([ms, ms_e2e], device='cuda', dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

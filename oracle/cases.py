@@ -1,5 +1,23 @@
 """Golden-case definitions shared by oracle/gen_golden.py and the tests (test infrastructure)."""
+import contextlib
+
 import torch
+
+# torch's CPU convolutions split their reductions by the number of intra-op threads, so the oracle reproduces the fixtures
+# bit-for-bit only at the thread count they were generated with
+GOLDEN_THREADS = 8
+
+
+@contextlib.contextmanager
+def golden_threads():
+    """Run torch's CPU ops with the thread count the fixtures were generated with."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(n)
+
 
 MINI = dict(depths=[1, 1, 2, 1], channels=[32, 64, 96, 128])
 MINI2 = dict(depths=[2, 2, 3, 2], channels=[32, 64, 128, 256])
@@ -87,6 +105,18 @@ def summarize_grad(g: torch.Tensor, full_below=4096, samples=256):
         return dict(full=g.clone())
     idx = torch.linspace(0, g.numel() - 1, samples).long()
     return dict(sample=g[idx].clone(), idx=idx, l2=g.double().norm().item(), s=g.double().sum().item())
+
+
+def assert_matches_summary(t: torch.Tensor, s: dict, what=''):
+    """t reproduces the tensor summarize_grad summarised as s bit-for-bit: every stored element equal, the full tensor's
+    float64 L2 norm and sum equal up to the summation order of the CPU kernels."""
+    t = t.detach().float().reshape(-1)
+    if 'full' in s:
+        assert torch.equal(t, s['full']), f'{what}: differs by {(t - s["full"]).abs().max()}'
+        return
+    assert torch.equal(t[s['idx']], s['sample']), f'{what}: sampled elements differ by {(t[s["idx"]] - s["sample"]).abs().max()}'
+    assert abs(t.double().norm().item() - s['l2']) <= 1e-12 * s['l2'], what
+    assert abs(t.double().sum().item() - s['s']) <= 1e-12 * s['l2'] * t.numel() ** 0.5, what
 
 
 # ---- LSKNet-MoE (BASELINE config 5 family; oracle/lsk_moe_oracle.py) --------------------------------------------

@@ -232,8 +232,8 @@ def run_lsk_case(name, spec):
 
 
 if __name__ == '__main__':
-    from oracle.cases import LSK_CASES
-    torch.set_num_threads(8)
+    from oracle.cases import GOLDEN_THREADS, LSK_CASES
+    torch.set_num_threads(GOLDEN_THREADS)
     names = sys.argv[1:] or (list(CASES) + list(LSK_CASES))
     for nm in names:
         if nm in LSK_CASES:

@@ -47,7 +47,7 @@ def test_backbone_refuses_cpu_input():
     (dict(arch='base', MoE_Block_inds=[[], [0, 2], list(range(0, 27, 2)), [0, 2]], num_experts=8, top_k=2), True),
 ])
 def test_state_dict_layout_matches_reference(kw, multi):
-    from oracle import ref_shim
+    from oracle import gen_reference_snapshots
     from oracle.convnext_moe_oracle import OracleConfig, param_shapes
     from sm3det_b200 import build_backbone
     name = 'ConvNeXt_moe_MultiInput' if multi else 'ConvNeXt_moe'
@@ -55,16 +55,16 @@ def test_state_dict_layout_matches_reference(kw, multi):
         net = build_backbone(dict(type=name, **kw))
     mine = {k: tuple(v.shape) for k, v in net.state_dict().items()}
     assert mine == param_shapes(OracleConfig(multi_input=multi, **kw))
-    if ref_shim.reference_available() and kw['arch'] == 'tiny':
-        ref = ref_shim.build_reference_backbone(name, **kw)      # the reference cannot be built on 'meta'
-        assert mine == {k: tuple(v.shape) for k, v in ref.state_dict().items()}
-        assert sorted(n for n, _ in net.named_parameters()) == sorted(n for n, _ in ref.named_parameters())
+    if kw['arch'] == 'tiny':          # recorded from the reference for the tiny cases (it cannot be built on 'meta')
+        ref, = [r for r in gen_reference_snapshots.load('convnext')['layouts'] if r['cls'] == name and r['kw'] == kw]
+        assert mine == ref['state_dict']
+        assert sorted(n for n, _ in net.named_parameters()) == sorted(ref['params'])
 
 
 def test_convnext_da_state_dict_and_shared_gate_weights():
     """ConvNeXt_DA_MultiInput (convnext_moe_DA.py): same keys, order and parameter names as the reference, including its quirk
     of ONE gate MLP registered under fc.0 / fc.1 / fc.2; the literal config dict of local_configs/main_DA_*.py builds."""
-    from oracle import ref_shim
+    from oracle import gen_reference_snapshots
     from oracle.convnext_moe_oracle import OracleConfig, param_shapes
     from sm3det_b200 import build_backbone
     kw = dict(arch='tiny', drop_path_rate=0.1, datasets=None)
@@ -75,10 +75,10 @@ def test_convnext_da_state_dict_and_shared_gate_weights():
     assert da.fc[0] is da.fc[1] is da.fc[2]
     names = [n for n, _ in net.named_parameters()]
     assert 'stages.0.0.DA.fc.0.0.weight' in names and 'stages.0.0.DA.fc.1.0.weight' not in names      # de-duplicated like the reference
-    if ref_shim.reference_available():
-        ref = ref_shim.build_reference_backbone('ConvNeXt_DA_MultiInput', module='convnext_moe_DA', **kw)
-        assert list(net.state_dict()) == list(ref.state_dict())
-        assert names == [n for n, _ in ref.named_parameters()]
+    ref = gen_reference_snapshots.load('convnext')['da_layout']      # recorded from the reference for these kwargs
+    assert ref['kw'] == kw
+    assert list(net.state_dict()) == list(ref['state_dict'])
+    assert names == ref['params']
     with pytest.raises(NotImplementedError):
         build_backbone(dict(type='ConvNeXt_DA_MultiInput', arch='tiny', datasets=['sar', 'rgb', 'ifr']))
 

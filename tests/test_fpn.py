@@ -1,10 +1,11 @@
-"""MultitaskFPN (next row, SURVEY 8f rank 1): oracle pinned against the unmodified reference (CPU), drop-in contract, and GPU
-parity of forward + every gradient (incl. the gradient flowing back into the 4 backbone maps) for the three call patterns the
-detector uses (trisource_H1stage_R2stage_detector.py:158-167)."""
+"""MultitaskFPN (next row, SURVEY 8f rank 1): oracle pinned against the unmodified reference's recorded outputs (CPU,
+oracle/gen_reference_snapshots.py), drop-in contract, and GPU parity of forward + every gradient (incl. the gradient flowing
+back into the 4 backbone maps) for the three call patterns the detector uses (trisource_H1stage_R2stage_detector.py:158-167)."""
 import pytest
 import torch
 
-from oracle import ref_shim
+from oracle import gen_reference_snapshots
+from oracle.cases import assert_matches_summary, golden_threads
 from oracle.fpn_oracle import fpn_forward, fpn_param_shapes
 from sm3det_b200.synth import make_state_dict
 
@@ -20,20 +21,19 @@ def _sd():
     return make_state_dict(fpn_param_shapes(KW['in_channels'], 256, 5, 1, 'on_output'), 5, True)
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason='reference tree not mounted')
 @pytest.mark.parametrize('start_level', [0, 1])
 def test_fpn_oracle_matches_reference(start_level):
-    mod = ref_shim.load_reference_module('Multitask_FPN', 'necks')
-    ref = mod.MultitaskFPN(**KW)
+    ref = gen_reference_snapshots.load('fpn')
+    assert ref['kw'] == KW
     sd = _sd()
-    assert set(sd) == set(ref.state_dict())
-    ref.load_state_dict(sd, strict=True)
+    assert set(sd) == set(ref['keys'])
     xs = _inputs()
-    with torch.no_grad():
-        r = ref(xs, start_level=start_level, add_extra_convs='on_output') if start_level else ref(xs)
+    with torch.no_grad(), golden_threads():
         o = fpn_forward(sd, xs, 4, 5, start_level, 'on_output')
+    r = ref['outs'][start_level]
     assert len(r) == len(o) == 5      # start_level=1 (SAR): 3 pyramid levels + 2 stride-2 extra levels
-    assert all(torch.equal(a, b) for a, b in zip(r, o))
+    for i, (a, b) in enumerate(zip(o, r)):
+        assert_matches_summary(a, b, f'level {i}')
 
 
 def test_fpn_contract():

@@ -309,7 +309,9 @@ def test_lsk_eval_list_input_and_plain_class():
 def test_fused_dropout(ops):
     """sm3_dropout: keep-rate ~ 1-p, survivors scaled by 1/(1-p), the backward reuses the identical mask, seeds differ."""
     from sm3det_b200.lsk_functional import DropoutFn
-    x = torch.randn(1 << 20, device='cuda').requires_grad_(True)
+    # seeded, and free of exact zeros (which would read as dropped below)
+    x = torch.randn(1 << 20, generator=torch.Generator().manual_seed(0)).cuda().requires_grad_(True)
+    assert bool((x != 0).all())
     y = DropoutFn.apply(x, 0.1, 1234)
     keep = (y != 0)
     assert abs(keep.float().mean().item() - 0.9) < 3e-3

@@ -1,18 +1,24 @@
 """CPU checks for the LSKNet-MoE family: oracle vs committed goldens (generated from the real reference by
-oracle/gen_golden.py), oracle vs the live reference when /root/reference is present, and the drop-in contract
-(state_dict keys / shapes, constructor kwargs) of the CUDA module -- no GPU compute."""
+oracle/gen_golden.py), oracle vs the reference's outputs and layouts recorded by oracle/gen_reference_snapshots.py, and the
+drop-in contract (state_dict keys / shapes, constructor kwargs) of the CUDA module -- no GPU compute."""
 import glob
 import os
 
 import pytest
 import torch
 
-from oracle import ref_shim
-from oracle.cases import LSK_CASES, lsk_injections
+from oracle import gen_reference_snapshots
+from oracle.cases import LSK_CASES, assert_matches_summary, golden_threads, lsk_injections
 from oracle.lsk_moe_oracle import LskConfig, lsk_backbone_forward, lsk_param_shapes
 from sm3det_b200.synth import make_images, make_state_dict
 
 GOLD = os.path.join(os.path.dirname(__file__), 'golden')
+
+
+@pytest.fixture(autouse=True)
+def _golden_threads():
+    with golden_threads():
+        yield
 
 
 def _inputs(gold):
@@ -45,21 +51,19 @@ def test_oracle_reproduces_reference_golden(path):
         assert torch.equal(bn[k], v), k
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason='reference tree not mounted')
 def test_oracle_matches_live_reference_lsk():
+    """Another image than the golden fixture; the reference's outputs were recorded from the live module."""
+    ref = gen_reference_snapshots.load('lsk')['live']
     spec = LSK_CASES['lsk_mini_moe_e4k2_eval']
     cfg = LskConfig(**spec['kw'])
-    mod = ref_shim.load_reference_module('lsk_moe')
-    torch.manual_seed(0)
-    net = mod.LSKNet_moe_MultiInput(norm_cfg=dict(type='SyncBN', requires_grad=True), **spec['kw'])
     sd = make_state_dict(lsk_param_shapes(cfg), 0, True)
-    net.load_state_dict(sd, strict=True)
-    net.eval()
     x = make_images(*spec['img'], seed=5)
     with torch.no_grad():
-        ref, rl = net(x)
         orc, ol = lsk_backbone_forward(sd, cfg, x, train=False)
-    assert all(torch.equal(a, b) for a, b in zip(ref, orc)) and torch.equal(rl, ol)
+    assert len(orc) == len(ref['outs'])
+    for i, (o, r) in enumerate(zip(orc, ref['outs'])):
+        assert_matches_summary(o, r, f'output {i}')
+    assert torch.equal(ol, ref['gate_loss'])
 
 
 def test_lsk_contract_state_dict_and_registry():
@@ -81,12 +85,11 @@ def test_lsk_contract_state_dict_and_registry():
     assert set(lsk_param_shapes(pc)) == set(plain.state_dict())
     with pytest.raises(RuntimeError):
         net(torch.zeros(1, 3, 64, 64))                    # CPU tensor: no fallback path
-    if ref_shim.reference_available():
-        mod = ref_shim.load_reference_module('lsk_moe')
-        ref = mod.LSKNet_moe_MultiInput(**kw)
-        assert set(ref.state_dict()) == set(sd)
-        up = {k: v for k, v in ref.state_dict().items()}
-        assert not net.load_state_dict(up, strict=True).missing_keys
+    ref = gen_reference_snapshots.load('lsk')['lsk_layout']
+    assert ref['kw'] == kw
+    assert set(ref['state_dict']) == set(sd)
+    up = {k: torch.zeros(shape, dtype=dtype) for k, (shape, dtype) in ref['state_dict'].items()}
+    assert not net.load_state_dict(up, strict=True).missing_keys
 
 
 def test_lsk_upcycle_dense_checkpoint():
@@ -147,9 +150,8 @@ def test_van_contract():
     shapes = lsk_param_shapes(LskConfig(spatial_unit='lka', **kw))
     sd = net.state_dict()
     assert set(shapes) == set(sd) and all(tuple(sd[k].shape) == tuple(v) for k, v in shapes.items())
-    if ref_shim.reference_available():
-        ref = ref_shim.load_reference_module('van_moe').VAN_moe_MultiInput(**kw)
-        assert set(ref.state_dict()) == set(sd)
+    ref = gen_reference_snapshots.load('lsk')['van_layout']
+    assert ref['kw'] == kw and set(ref['keys']) == set(sd)
 
 
 def test_forced_channel_argmax_is_identity_on_own_choice():

@@ -1,18 +1,24 @@
 """The CPU oracle against (a) the committed golden fixtures generated from the unmodified reference
-and (b) the live reference module when /root/reference is present (build container only)."""
+and (b) the reference modules' own outputs recorded by oracle/gen_reference_snapshots.py."""
 import glob
 import os
 
 import pytest
 import torch
 
-from oracle import ref_shim
-from oracle.cases import CASES, make_noise, summarize_grad, upstream_grads
+from oracle import gen_reference_snapshots
+from oracle.cases import CASES, assert_matches_summary, golden_threads, make_noise, summarize_grad, upstream_grads
 from oracle.convnext_moe_oracle import OracleConfig, backbone_forward, param_shapes, tie_da_weights
 from oracle.gen_golden import moe_token_counts
 from sm3det_b200.synth import make_images, make_state_dict, state_dict_checksum
 
 GOLD = os.path.join(os.path.dirname(__file__), 'golden')
+
+
+@pytest.fixture(autouse=True)
+def _golden_threads():
+    with golden_threads():
+        yield
 
 
 def _run_oracle(gold, record):
@@ -76,40 +82,36 @@ def test_oracle_matches_reference_golden(path):
                 assert abs(s['l2'] - g['l2']) <= 1e-5 * (g['l2'] + 1e-12)
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason='/root/reference not mounted')
 @pytest.mark.parametrize('name', ['mini_moe_e4k2_eval', 'mini_moe_e8k3_eval'])
 def test_oracle_matches_live_reference(name):
+    """Another weight seed and image than the golden fixture; the reference's outputs were recorded from the live module."""
+    ref = gen_reference_snapshots.load('convnext')['live'][name]
     spec = CASES[name]
     kw = dict(spec['kw'])
     cfg = OracleConfig(**kw)
-    net = ref_shim.build_reference_backbone('ConvNeXt_moe_MultiInput', seed=0, **kw)
     sd = make_state_dict(param_shapes(cfg), 3, True)
-    net.load_state_dict(sd, strict=True)
-    net.eval()
     x = make_images(2, 64, 64, seed=5)
     with torch.no_grad():
-        ref = net(x)
-        orc = backbone_forward(sd, cfg, x)
-    for a, b in zip(ref[0], orc[0]):
-        assert torch.equal(a, b)
-    assert torch.equal(ref[1], orc[1])
+        outs, loss = backbone_forward(sd, cfg, x)
+    assert len(outs) == len(ref['outs'])
+    for i, (o, r) in enumerate(zip(outs, ref['outs'])):
+        assert_matches_summary(o, r, f'output {i}')
+    assert torch.equal(loss, ref['gate_loss'])
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason='/root/reference not mounted')
 def test_plain_convnext_moe_class_matches():
     """ConvNeXt_moe (stem inside downsample_layers.0) -- convnext_moe.py:407-600."""
+    ref = gen_reference_snapshots.load('convnext')['plain']
     kw = dict(arch=dict(depths=[1, 1, 2, 1], channels=[32, 64, 96, 128]), MoE_Block_inds=[[], [], [1], []],
               num_experts=4, top_k=2)
+    assert ref['kw'] == kw
     cfg = OracleConfig(multi_input=False, **kw)
-    net = ref_shim.build_reference_backbone('ConvNeXt_moe', seed=0, **kw)
     shapes = param_shapes(cfg)
-    assert set(shapes) == set(net.state_dict())
+    assert set(shapes) == set(ref['keys'])
     sd = make_state_dict(shapes, 1, True)
-    net.load_state_dict(sd, strict=True)
-    net.eval()
     x = make_images(1, 64, 64, seed=2)
     with torch.no_grad():
-        ref = net(x)
-        orc = backbone_forward(sd, cfg, x)
-    for a, b in zip(ref[0], orc[0]):
-        assert torch.equal(a, b)
+        outs = backbone_forward(sd, cfg, x)[0]
+    assert len(outs) == len(ref['outs'])
+    for i, (o, r) in enumerate(zip(outs, ref['outs'])):
+        assert_matches_summary(o, r, f'output {i}')
