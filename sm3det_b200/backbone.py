@@ -158,22 +158,9 @@ class ConvNeXtBlock(nn.Module):
         self._packs.invalidate()
         return super()._load_from_state_dict(*args, **kwargs)
 
-    def _row_scale(self, x):
-        """timm DropPath as a per-token scale (per-sample Bernoulli(keep) / keep), None when inactive."""
-        if self.drop_path_rate == 0. or not self.training:
-            return None
-        keep = 1.0 - self.drop_path_rate
-        N, H, W, _ = x.shape
-        mask = getattr(self, '_injected_drop_mask', None)
-        if mask is None:
-            mask = x.new_empty((N,)).bernoulli_(keep)
-            if keep > 0.0:
-                mask = mask / keep
-        return mask.to(x.device, torch.float32).repeat_interleave(H * W).contiguous()
-
     def forward(self, x, record=None):
         """x: NHWC fp32.  Returns (x, loss) like the reference block (:343-379); loss is None if dense."""
-        return self._run(x, self._row_scale(x), record, True)
+        return self._run(x, Fn.drop_path_row_scale(self, x), record, True)
 
     def _run(self, x, rs, record, shortcut):
         """shortcut=False returns the branch rs * gamma * ffn(norm(dwconv(x))) without the residual add (ConvNeXt_DA)."""
@@ -200,13 +187,7 @@ class ConvNeXtBlock(nn.Module):
                                         w1, f.pointwise_conv1.bias, w2, f.pointwise_conv2.bias, self.gamma, rs, eps, packs)
             return out, None
         m = self.ffn
-        noise = None
-        if m.noisy_gating and self.training:
-            noise = getattr(m, '_injected_noise', None)
-            if noise is None:
-                T = x.shape[0] * x.shape[1] * x.shape[2]
-                noise = torch.randn((T, m.num_experts), device=x.device, dtype=torch.float32)
-            noise = noise.to(x.device, torch.float32).contiguous()
+        noise = Fn.gating_noise(m, x.shape[0] * x.shape[1] * x.shape[2], x.device)
         g = m.w_gate
         ep = m.expert_params()
         E = m.num_experts
@@ -271,7 +252,7 @@ class ConvNeXtDABlock(ConvNeXtBlock):
         self.DA = DALayer(self.gamma.shape[0])
 
     def forward(self, x, record=None, datasets=('rgb',)):
-        rs = self._row_scale(x)
+        rs = Fn.drop_path_row_scale(self, x)
         y, loss = self._run(x, None, record, False)        # gamma * ffn(norm(dwconv(x))), NHWC
         s = self.DA.gate(Fn.SampleMeanFn.apply(y), list(datasets))
         return Fn.DAGateFn.apply(y, x, s, rs), loss

@@ -210,9 +210,7 @@ class EPMoEBlockFn(Function):
         u = ops.dwconv7(x, Fn._taps(dww), dwb)
         v = B['v'].view(T, C)
         _, stats = ops.layernorm_fwd(u, lnw, lnb, eps, tokens=T, C=C, out=v, save_stats=train)
-        r = ops.moe_router(v, wp, bp, sim, tau, T=T, Cc=C, E=E, k=k, w_noise=w_noise, noise=noise, save=train)
-        plan = ops.moe_plan(r['partials'], T=T, E=E, k=k)
-        slot_of, pair_token = ops.moe_assign(r['top_idx'], plan, T=T, E=E, k=k)
+        r, plan, slot_of, pair_token = Fn.route(v, wp, bp, sim, tau, w_noise, noise, T=T, C=C, E=E, k=k, save=train)
         R_s, cap = plan['max_rows'], B['cap']
         B['pair'][:R_s].copy_(pair_token)
         meta = torch.stack([plan['counts'], plan['seg_begin']]).contiguous()
@@ -222,11 +220,8 @@ class EPMoEBlockFn(Function):
         grouped = (P['tile_group'], P['num_tiles'])
         # every expert-side kernel runs over the fixed `cap` row space; the live tile count / segments come from the device
         xr = ops.gather_rows_peer(B['v_ptrs'], P['src_rank'], P['src_slot'], rows=cap, Cc=C, token_lists=B['pair_ptrs'])
-        h = ops.linear_fwd(xr, w1s[own], b1s[own], rows=cap, grouped=grouped, w_group_stride=4 * C * C,
-                           bias_group_stride=4 * C, packed=packs.get('w1'))
-        a_k, _, _ = ops.act_pack(h, rows=cap, width=4 * C, mode=ops.ACT_GELU, want_k=True, live_tiles=P['num_tiles'])
-        ops.linear_fwd(None, w2s[own], b2s[own], rows=cap, a_packed=a_k, grouped=grouped, w_group_stride=4 * C * C,
-                       bias_group_stride=C, packed=packs.get('w2'), out=B['o'][:cap * C].view(cap, C))
+        h, _ = Fn.expert_ffn_fwd(xr, w1s[own], b1s[own], w2s[own], b2s[own], packs, rows=cap, grouped=grouped,
+                                 out=B['o'][:cap * C].view(cap, C))
         ep.barrier()                                                 # every rank's expert outputs are complete
         o = ops.gather_rows_peer(B['o_ptrs'], P['comb_rank'], P['comb_row'], rows=R_s, Cc=C)
         out, y = ops.moe_combine(o, slot_of, r['top_idx'], r['top_gate'], gamma, x.view(T, C), row_scale, T=T, Cc=C, k=k,
@@ -235,20 +230,20 @@ class EPMoEBlockFn(Function):
             record.append(dict(v=v.clone(), top_idx=r['top_idx'], top_gate=r['top_gate'], importance=plan['importance'],
                                load=plan['load'], loss=plan['loss'], y=y, counts=plan['counts']))
         if train:
-            ctx.noisy = noise is not None     # gates depend on w_noise whenever noise was added, also for k == E
-            ctx.save_for_backward(x, u, stats, v.clone(), h, xr, o, dww, lnw, gamma, wp, sim, tau, row_scale, r['top_idx'],
-                                  r['top_gate'], r['logits'], r['p'], slot_of, plan['importance'], w1s[own], w2s[own], noise,
-                                  r['sigma'], r['top_vals'], r['top_idx_m'], plan['load'], w_noise)
+            # v lives in the symmetric buffer that the next layer of this shape overwrites: save a copy
+            ctx.save_for_backward(*Fn.router_saved(r, plan, sim, tau, noise, w_noise), x, u, stats, v.clone(), h, xr, o, dww,
+                                  lnw, gamma, wp, row_scale, slot_of, w1s[own], w2s[own])
             ctx.P, ctx.B, ctx.ep = P, B, ep
             ctx.E, ctx.k, ctx.R_s, ctx.own, ctx.E_loc = E, k, R_s, own, E_loc
             ctx.packs = packs
-            ctx.has_noise_param = w_noise is not None
         return out.view(N, H, W_, C), plan['loss'].reshape(())
 
     @staticmethod
     def backward(ctx, dout, dloss):
-        (x, u, stats, v, h, xr, o, dww, lnw, gamma, wp, sim, tau, rs, top_idx, top_gate, logits, p, slot_of, importance,
-         w1, w2, noise, sigma, top_vals, top_idx_m, load, w_noise) = ctx.saved_tensors
+        saved = ctx.saved_tensors
+        router = saved[:Fn.ROUTER_SAVED]
+        x, u, stats, v, h, xr, o, dww, lnw, gamma, wp, rs, slot_of, w1, w2 = saved[Fn.ROUTER_SAVED:]
+        top_idx, top_gate = router[:2]
         P, B, ep = ctx.P, ctx.B, ctx.ep
         E, k, R_s, own, E_loc = ctx.E, ctx.k, ctx.R_s, ctx.own, ctx.E_loc
         N, H, W_, C = x.shape
@@ -265,50 +260,14 @@ class EPMoEBlockFn(Function):
         dgate = ops.moe_combine_bwd(dz, o, slot_of, top_idx, top_gate, gamma, rs, d_o, dgamma, T=T, Cc=C, k=k)
         ep.barrier()                                                 # every rank's d_o rows are complete
         # gradients exist for the OWNED experts only (the others return None and stay out of the DDP buckets)
-        dw1s = torch.zeros((E_loc, 4 * C, C), device=dev, dtype=torch.float32)
-        db1s = torch.zeros((E_loc, 4 * C), device=dev, dtype=torch.float32)
-        dw2s = torch.zeros((E_loc, C, 4 * C), device=dev, dtype=torch.float32)
-        db2s = torch.zeros((E_loc, C), device=dev, dtype=torch.float32)
         dor = ops.gather_rows_peer(B['do_ptrs'], P['src_rank'], P['src_slot'], rows=cap, Cc=C)
-        da = ops.linear_dgrad(dor, w2, grouped=grouped, w_group_stride=4 * C * C, packed=ctx.packs.get('w2_t'))
-        # one pass over h: dh = da * gelu'(h) as dgrad1's / wgrad1's operands (+ db1) and a = gelu(h) as wgrad2's operand
-        dh_k, dh_mn, a_mn = ops.act_pack(h, rows=cap, width=4 * C, mode=ops.ACT_BWD, da=da, want_k=True, mn_tile=128,
-                                      mn_tile2=ops._pick_bn(4 * C), colsum=db1s, live_tiles=P['num_tiles'], tile_group=P['tile_group'])
-        del da
-        ops.linear_wgrad(dor, None, dw2s, rows=cap, segs=segs, num_groups=E_loc, x_packed=a_mn)
-        del a_mn
-        ops.colsum(dor, db2s, rows=cap, Cc=C, segs=segs, groups=E_loc)
-        ops.linear_wgrad(None, xr, dw1s, rows=cap, segs=segs, num_groups=E_loc, dy_packed=dh_mn)
-        dxp = B['dxp'][:cap * C].view(cap, C)
-        ops.linear_dgrad(None, w1, rows=cap, a_packed=dh_k, out=dxp, grouped=grouped, w_group_stride=4 * C * C,
-                         packed=ctx.packs.get('w1_t'))
+        dxp, dw1s, db1s, dw2s, db2s = Fn.expert_ffn_bwd(dor, h, xr, w1, w2, ctx.packs, rows=cap, grouped=grouped, segs=segs,
+                                                        groups=E_loc, dxp=B['dxp'][:cap * C].view(cap, C))
         ep.barrier()                                                 # every rank's d_x rows are complete
         dxp_l = ops.gather_rows_peer(B['dxp_ptrs'], P['comb_rank'], P['comb_row'], rows=R_s, Cc=C)
-        # router (local)
-        Pp = wp.shape[0]
-        dtau = torch.zeros((1,), device=dev, dtype=torch.float32)
-        dsim = torch.zeros((Pp, E), device=dev, dtype=torch.float32)
-        lscale = dloss.reshape(1).contiguous().float()
-        noisy = dict(noise=noise, sigma=sigma, top_vals=top_vals, top_idx_m=top_idx_m, load=load) if ctx.noisy else None
-        dp, dr = ops.moe_router_bwd(p, sim, tau, top_idx, top_gate, dgate, logits, importance, lscale, dsim, dtau, T=T, E=E,
-                                    k=k, noisy=noisy)
-        dwp = torch.zeros_like(wp)
-        ops.linear_wgrad(dp, v, dwp)
-        dbp = torch.zeros((Pp,), device=dev, dtype=torch.float32)
-        ops.colsum(dp, dbp, rows=T, Cc=Pp)
-        dv_r = ops.linear_dgrad(dp, wp, packed=ctx.packs.get('wp_t'))
-        dwn = None
-        if ctx.noisy:
-            wn_t = torch.zeros((32, C), device=dev, dtype=torch.float32)
-            wn_t[:E] = w_noise.t()
-            dwn_t = torch.zeros((32, C), device=dev, dtype=torch.float32)
-            ops.linear_wgrad(dr, v, dwn_t)
-            dwn = dwn_t[:E].t().contiguous()
-            dv_r = ops.linear_dgrad(dr, wn_t, epilogue=ops.EPI_RESID, resid=dv_r)
+        dv_r, dwp, dbp, dsim, dtau, dwn = Fn.router_backward(router, v, wp, dgate, dloss, ctx.packs.get('wp_t'))
         dv = ops.gather_sum(dxp_l, slot_of, dv_r, T=T, Cc=C, k=k)
         dx, ddww, ddwb, dlnw, dlnb = Fn._block_front_bwd(dv, dout, x, u, stats, dww, lnw)
-        if dwn is None and ctx.has_noise_param:
-            dwn = torch.zeros((C, E), device=dev, dtype=torch.float32)
         if ep.average_grads:                  # what DDP's mean over ranks does to every other gradient
             for t in (dw1s, db1s, dw2s, db2s):
                 t.mul_(1.0 / ep.world)

@@ -23,12 +23,12 @@ def _zeros_like_param(p):
     return torch.zeros(p.shape, device=p.device, dtype=torch.float32)
 
 
-def _taps(dww):            # [C,1,7,7] -> [49][C]
-    return dww.reshape(dww.shape[0], 49).t().contiguous()
+def _taps(w):              # [C,1,ks,ks] -> [ks*ks][C]
+    return w.reshape(w.shape[0], -1).t().contiguous()
 
 
-def _taps_flipped(dww):    # correlation taps for dgrad
-    return dww.flip(2, 3).reshape(dww.shape[0], 49).t().contiguous()
+def _taps_flipped(w):      # correlation taps for dgrad
+    return w.flip(2, 3).reshape(w.shape[0], -1).t().contiguous()
 
 
 @ops.captures_precision
@@ -253,6 +253,121 @@ def stack_expert_params(params):
             p.data = flat[i]
 
 
+def gating_noise(layer, T, device):
+    """[T, E] gating noise of a noisy-gating MoE layer in training, else None (tests inject ``_injected_noise``)."""
+    if not (layer.noisy_gating and layer.training):
+        return None
+    noise = getattr(layer, '_injected_noise', None)
+    if noise is None:
+        noise = torch.randn((T, layer.num_experts), device=device, dtype=torch.float32)
+    return noise.to(device, torch.float32).contiguous()
+
+
+def drop_path_row_scale(block, x):
+    """timm DropPath as a per-token scale of NHWC x (per-sample Bernoulli(keep) / keep), None when inactive.
+    Tests inject the per-sample mask as ``_injected_drop_mask``."""
+    if block.drop_path_rate == 0. or not block.training:
+        return None
+    keep = 1.0 - block.drop_path_rate
+    N, H, W, _ = x.shape
+    mask = getattr(block, '_injected_drop_mask', None)
+    if mask is None:
+        mask = x.new_empty((N,)).bernoulli_(keep)
+        if keep > 0.0:
+            mask = mask / keep
+    return mask.to(x.device, torch.float32).repeat_interleave(H * W).contiguous()
+
+
+def route(v, wp, bp, sim, tau, w_noise, noise, *, T, C, E, k, save):
+    """Router -> plan -> slot assignment of one MoE layer: (r, plan, slot_of, pair_token)."""
+    r = ops.moe_router(v, wp, bp, sim, tau, T=T, Cc=C, E=E, k=k, w_noise=w_noise, noise=noise, save=save)
+    plan = ops.moe_plan(r['partials'], T=T, E=E, k=k)
+    slot_of, pair_token = ops.moe_assign(r['top_idx'], plan, T=T, E=E, k=k)
+    return r, plan, slot_of, pair_token
+
+
+ROUTER_SAVED = 13      # number of tensors router_saved returns
+
+
+def router_saved(r, plan, sim, tau, noise, w_noise):
+    """The tensors router_backward needs, in its order; top_idx and top_gate come first (combine backward uses them)."""
+    return (r['top_idx'], r['top_gate'], r['p'], sim, tau, r['logits'], plan['importance'], noise, r['sigma'],
+            r['top_vals'], r['top_idx_m'], plan['load'], w_noise)
+
+
+def router_backward(saved, v, wp, dgate, dloss, wp_t=None):
+    """(dv_r, dwp, dbp, dsim, dtau, dwn) of the router that saw the rows v [T, C]; ``saved`` is router_saved(...).
+    The gates depend on w_noise whenever noise was drawn, also for k == E.  Without noise dwn is zero (DDP wants a
+    gradient for every parameter), None if the layer has no w_noise."""
+    top_idx, top_gate, p, sim, tau, logits, importance, noise, sigma, top_vals, top_idx_m, load, w_noise = saved
+    T, C = v.shape
+    P, E = sim.shape
+    k = top_idx.shape[1]
+    dev = v.device
+    dtau = torch.zeros((1,), device=dev, dtype=torch.float32)
+    dsim = torch.zeros((P, E), device=dev, dtype=torch.float32)
+    lscale = dloss.reshape(1).contiguous().float()
+    noisy = None if noise is None else dict(noise=noise, sigma=sigma, top_vals=top_vals, top_idx_m=top_idx_m, load=load)
+    dp, dr = ops.moe_router_bwd(p, sim, tau, top_idx, top_gate, dgate, logits, importance, lscale, dsim, dtau, T=T,
+                                E=E, k=k, noisy=noisy)
+    dwp = torch.zeros_like(wp)
+    ops.linear_wgrad(dp, v, dwp)
+    dbp = torch.zeros((P,), device=dev, dtype=torch.float32)
+    ops.colsum(dp, dbp, rows=T, Cc=P)
+    dv_r = ops.linear_dgrad(dp, wp, packed=wp_t)
+    dwn = None
+    if noise is not None:
+        # r = v @ w_noise is an [T,C]x[C,E] product with E < 32: run it as a 32-wide zero-padded GEMM pair
+        wn_t = torch.zeros((32, C), device=dev, dtype=torch.float32)
+        wn_t[:E] = w_noise.t()
+        dwn_t = torch.zeros((32, C), device=dev, dtype=torch.float32)
+        ops.linear_wgrad(dr, v, dwn_t)                             # [32,C] = dr^T v
+        dwn = dwn_t[:E].t().contiguous()
+        dv_r = ops.linear_dgrad(dr, wn_t, epilogue=EPI_RESID, resid=dv_r)
+    elif w_noise is not None:
+        dwn = torch.zeros((C, E), device=dev, dtype=torch.float32)
+    return dv_r, dwp, dbp, dsim, dtau, dwn
+
+
+def expert_ffn_fwd(a, w1, b1, w2, b2, packs, *, rows, grouped, row_index=None, out=None):
+    """Grouped two-GEMM experts over ``rows`` expert-sorted rows: h = a[row_index] w1^T + b1 (no row_index: a is in
+    expert order already), o = gelu(h) w2^T + b2 (into ``out`` when given).  w1 .. b2 are the first expert's stacked
+    parameters (stack_expert_params).  Returns (h, o)."""
+    C = a.shape[1]
+    h = ops.linear_fwd(a, w1, b1, row_index=row_index, rows=rows, grouped=grouped, w_group_stride=4 * C * C,
+                       bias_group_stride=4 * C, packed=packs.get('w1'))
+    a_k, _, _ = ops.act_pack(h, rows=rows, width=4 * C, mode=ops.ACT_GELU, want_k=True, live_tiles=grouped[1])
+    o = ops.linear_fwd(None, w2, b2, rows=rows, a_packed=a_k, grouped=grouped, w_group_stride=4 * C * C,
+                       bias_group_stride=C, packed=packs.get('w2'), out=out)
+    return h, o
+
+
+def expert_ffn_bwd(d_o, h, a, w1, w2, packs, *, rows, grouped, segs, groups, row_index=None, dxp=None):
+    """Backward of expert_ffn_fwd: (dxp, dw1s, db1s, dw2s, db2s), weight gradients stacked over ``groups`` experts.
+    dxp (the given buffer, or a new one) is written at every live row; padding rows are never read."""
+    C = a.shape[1]
+    dev = d_o.device
+    da = ops.linear_dgrad(d_o, w2, grouped=grouped, w_group_stride=4 * C * C, packed=packs.get('w2_t'))
+    db1s = torch.zeros((groups, 4 * C), device=dev, dtype=torch.float32)
+    # one pass over h: dh = da * gelu'(h) as dgrad1's / wgrad1's operands (+ db1) and a = gelu(h) as wgrad2's operand
+    dh_k, dh_mn, a_mn = ops.act_pack(h, rows=rows, width=4 * C, mode=ops.ACT_BWD, da=da, want_k=True, mn_tile=128,
+                                     mn_tile2=ops._pick_bn(4 * C), colsum=db1s, live_tiles=grouped[1],
+                                     tile_group=grouped[0])
+    del da
+    dw2s = torch.zeros((groups, C, 4 * C), device=dev, dtype=torch.float32)
+    ops.linear_wgrad(d_o, None, dw2s, rows=rows, segs=segs, num_groups=groups, x_packed=a_mn)
+    del a_mn
+    db2s = torch.zeros((groups, C), device=dev, dtype=torch.float32)
+    ops.colsum(d_o, db2s, rows=rows, Cc=C, segs=segs, groups=groups)
+    dw1s = torch.zeros((groups, 4 * C, C), device=dev, dtype=torch.float32)
+    ops.linear_wgrad(None, a, dw1s, rows=rows, x_row_index=row_index, segs=segs, num_groups=groups, dy_packed=dh_mn)
+    if dxp is None:
+        dxp = torch.empty((rows, C), device=dev, dtype=torch.float32)
+    ops.linear_dgrad(None, w1, rows=rows, a_packed=dh_k, out=dxp, grouped=grouped, w_group_stride=4 * C * C,
+                     packed=packs.get('w1_t'))
+    return dxp, dw1s, db1s, dw2s, db2s
+
+
 @ops.captures_precision
 class MoEBlockFn(Function):
     """x -> dwconv -> LN -> router/plan/assign -> grouped expert GEMMs -> combine (+gamma, +shortcut)."""
@@ -265,16 +380,10 @@ class MoEBlockFn(Function):
         w1s, b1s, w2s, b2s = experts[0:E], experts[E:2 * E], experts[2 * E:3 * E], experts[3 * E:4 * E]
         train = any(ctx.needs_input_grad)
         u, v, stats = _block_front(x, dww, dwb, lnw, lnb, eps, train)
-        r = ops.moe_router(v, wp, bp, sim, tau, T=T, Cc=C, E=E, k=k, w_noise=w_noise, noise=noise, save=train)
-        plan = ops.moe_plan(r['partials'], T=T, E=E, k=k)
-        slot_of, pair_token = ops.moe_assign(r['top_idx'], plan, T=T, E=E, k=k)
+        r, plan, slot_of, pair_token = route(v, wp, bp, sim, tau, w_noise, noise, T=T, C=C, E=E, k=k, save=train)
         R = plan['max_rows']
-        grouped = (plan['tile_group'], plan['num_m_tiles'])
-        h = ops.linear_fwd(v, w1s[0], b1s[0], row_index=pair_token, rows=R, grouped=grouped, w_group_stride=4 * C * C,
-                           bias_group_stride=4 * C, packed=packs.get('w1'))
-        a_k, _, _ = ops.act_pack(h, rows=R, width=4 * C, mode=ops.ACT_GELU, want_k=True, live_tiles=plan['num_m_tiles'])
-        o = ops.linear_fwd(None, w2s[0], b2s[0], rows=R, a_packed=a_k, grouped=grouped, w_group_stride=4 * C * C,
-                           bias_group_stride=C, packed=packs.get('w2'))
+        h, o = expert_ffn_fwd(v, w1s[0], b1s[0], w2s[0], b2s[0], packs, rows=R,
+                              grouped=(plan['tile_group'], plan['num_m_tiles']), row_index=pair_token)
         ctx.shortcut = packs.get('shortcut', True)
         out, y = ops.moe_combine(o, slot_of, r['top_idx'], r['top_gate'], gamma, x.view(T, C) if ctx.shortcut else None,
                                  row_scale, T=T, Cc=C, k=k, want_y=record is not None)
@@ -282,77 +391,36 @@ class MoEBlockFn(Function):
             record.append(dict(v=v, top_idx=r['top_idx'], top_gate=r['top_gate'], importance=plan['importance'],
                                load=plan['load'], loss=plan['loss'], y=y, counts=plan['counts']))
         if train:
-            ctx.noisy = noise is not None     # gates depend on w_noise whenever noise was added, also for k == E
-            ctx.save_for_backward(x, u, stats, v, h, o, dww, lnw, gamma, wp, sim, tau, row_scale, r['top_idx'],
-                                  r['top_gate'], r['logits'], r['p'], slot_of, pair_token, plan['importance'],
-                                  plan['seg_begin'], plan['seg_end'], plan['tile_group'], plan['num_m_tiles'],
-                                  w1s[0], w2s[0], noise, r['sigma'], r['top_vals'], r['top_idx_m'], plan['load'],
-                                  w_noise)
+            ctx.save_for_backward(*router_saved(r, plan, sim, tau, noise, w_noise), x, u, stats, v, h, o, dww, lnw, gamma,
+                                  wp, row_scale, slot_of, pair_token, plan['seg_begin'], plan['seg_end'],
+                                  plan['tile_group'], plan['num_m_tiles'], w1s[0], w2s[0])
             ctx.E, ctx.k, ctx.R = E, k, R
             ctx.packs = packs
-            ctx.has_noise_param = w_noise is not None
         return out.view(N, H, W, C), plan['loss'].reshape(())
 
     @staticmethod
     def backward(ctx, dout, dloss):
-        (x, u, stats, v, h, o, dww, lnw, gamma, wp, sim, tau, rs, top_idx, top_gate, logits, p, slot_of, pair_token,
-         importance, seg_begin, seg_end, tile_group, num_m_tiles, w1, w2, noise, sigma, top_vals, top_idx_m, load,
-         w_noise) = ctx.saved_tensors
+        saved = ctx.saved_tensors
+        router = saved[:ROUTER_SAVED]
+        (x, u, stats, v, h, o, dww, lnw, gamma, wp, rs, slot_of, pair_token, seg_begin, seg_end, tile_group, num_m_tiles,
+         w1, w2) = saved[ROUTER_SAVED:]
+        top_idx, top_gate = router[:2]
         E, k, R = ctx.E, ctx.k, ctx.R
         N, H, W, C = x.shape
         T = N * H * W
         dev = x.device
         dout = dout.contiguous()
         dz = dout.view(T, C)
-        grouped = (tile_group, num_m_tiles)
-        segs = (seg_begin, seg_end)
         # combine / layer scale / shortcut
         d_o = torch.zeros((R, C), device=dev, dtype=torch.float32)
         dgamma = torch.zeros((C,), device=dev, dtype=torch.float32)
         dgate = ops.moe_combine_bwd(dz, o, slot_of, top_idx, top_gate, gamma, rs, d_o, dgamma, T=T, Cc=C, k=k)
         # experts (grouped over the padded expert segments)
-        da = ops.linear_dgrad(d_o, w2, grouped=grouped, w_group_stride=4 * C * C, packed=ctx.packs.get('w2_t'))
-        db1s = torch.zeros((E, 4 * C), device=dev, dtype=torch.float32)
-        # one pass over h: dh = da * gelu'(h) as dgrad1's / wgrad1's operands (+ db1) and a = gelu(h) as wgrad2's operand
-        dh_k, dh_mn, a_mn = ops.act_pack(h, rows=R, width=4 * C, mode=ops.ACT_BWD, da=da, want_k=True, mn_tile=128,
-                                      mn_tile2=ops._pick_bn(4 * C), colsum=db1s, live_tiles=num_m_tiles, tile_group=tile_group)
-        del da
-        dw2s = torch.zeros((E, C, 4 * C), device=dev, dtype=torch.float32)
-        ops.linear_wgrad(d_o, None, dw2s, rows=R, segs=segs, num_groups=E, x_packed=a_mn)
-        del a_mn
-        db2s = torch.zeros((E, C), device=dev, dtype=torch.float32)
-        ops.colsum(d_o, db2s, rows=R, Cc=C, segs=segs, groups=E)
-        dw1s = torch.zeros((E, 4 * C, C), device=dev, dtype=torch.float32)
-        ops.linear_wgrad(None, v, dw1s, rows=R, x_row_index=pair_token, segs=segs, num_groups=E, dy_packed=dh_mn)
-        dxp = torch.empty((R, C), device=dev, dtype=torch.float32)   # every row gather_sum reads (live slots) is written by the GEMM
-        ops.linear_dgrad(None, w1, rows=R, a_packed=dh_k, out=dxp, grouped=grouped, w_group_stride=4 * C * C,
-                         packed=ctx.packs.get('w1_t'))
-        # router
-        P = wp.shape[0]
-        dtau = torch.zeros((1,), device=dev, dtype=torch.float32)
-        dsim = torch.zeros((P, E), device=dev, dtype=torch.float32)
-        lscale = dloss.reshape(1).contiguous().float()
-        noisy = dict(noise=noise, sigma=sigma, top_vals=top_vals, top_idx_m=top_idx_m, load=load) if ctx.noisy else None
-        dp, dr = ops.moe_router_bwd(p, sim, tau, top_idx, top_gate, dgate, logits, importance, lscale, dsim, dtau, T=T,
-                                    E=E, k=k, noisy=noisy)
-        dwp = torch.zeros_like(wp)
-        ops.linear_wgrad(dp, v, dwp)
-        dbp = torch.zeros((P,), device=dev, dtype=torch.float32)
-        ops.colsum(dp, dbp, rows=T, Cc=P)
-        dv_r = ops.linear_dgrad(dp, wp, packed=ctx.packs.get('wp_t'))
-        dwn = None
-        if ctx.noisy:
-            # r = v @ w_noise is an [T,C]x[C,E] product with E < 32: run it as a 32-wide zero-padded GEMM pair
-            wn_t = torch.zeros((32, C), device=dev, dtype=torch.float32)
-            wn_t[:E] = w_noise.t()
-            dwn_t = torch.zeros((32, C), device=dev, dtype=torch.float32)
-            ops.linear_wgrad(dr, v, dwn_t)                             # [32,C] = dr^T v
-            dwn = dwn_t[:E].t().contiguous()
-            dv_r = ops.linear_dgrad(dr, wn_t, epilogue=EPI_RESID, resid=dv_r)
+        dxp, dw1s, db1s, dw2s, db2s = expert_ffn_bwd(d_o, h, v, w1, w2, ctx.packs, rows=R, grouped=(tile_group, num_m_tiles),
+                                                     segs=(seg_begin, seg_end), groups=E, row_index=pair_token)
+        dv_r, dwp, dbp, dsim, dtau, dwn = router_backward(router, v, wp, dgate, dloss, ctx.packs.get('wp_t'))
         dv = ops.gather_sum(dxp, slot_of, dv_r, T=T, Cc=C, k=k)
         dx, ddww, ddwb, dlnw, dlnb = _block_front_bwd(dv, dout if ctx.shortcut else None, x, u, stats, dww, lnw)
-        if dwn is None and ctx.has_noise_param:
-            dwn = torch.zeros((C, E), device=dev, dtype=torch.float32)
         grads_e = [dw1s[e] for e in range(E)] + [db1s[e] for e in range(E)] + [dw2s[e] for e in range(E)] + \
                   [db2s[e] for e in range(E)]
         return (dx, ddww, ddwb, dlnw, dlnb, dgamma, dwp, dbp, dsim, dtau, dwn, None, None, None, None, None, None, None,

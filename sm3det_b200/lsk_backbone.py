@@ -82,13 +82,7 @@ class MoE_layer(nn.Module):
         return ws + bs
 
     def forward(self, x, gamma=None, resid=None, row_scale=None, record=None):
-        noise = None
-        if self.noisy_gating and self.training:
-            noise = getattr(self, '_injected_noise', None)
-            if noise is None:
-                T = x.numel() // x.shape[-1]
-                noise = torch.randn((T, self.num_experts), device=x.device, dtype=torch.float32)
-            noise = noise.to(x.device, torch.float32).contiguous()
+        noise = Fn.gating_noise(self, x.numel() // x.shape[-1], x.device)
         g = self.w_gate
         return LF.MoELinearFn.apply(x, g.cosine_projector.weight, g.cosine_projector.bias, g.sim_matrix, g.temperature,
                                     self.w_noise, noise, gamma, resid, row_scale, self.num_experts, self.k, record,
@@ -237,24 +231,12 @@ class Block(nn.Module):
         self.layer_scale_1 = nn.Parameter(layer_scale_init_value * torch.ones((dim)), requires_grad=True)
         self.layer_scale_2 = nn.Parameter(layer_scale_init_value * torch.ones((dim)), requires_grad=True)
 
-    def _row_scale(self, x):
-        if self.drop_path_rate == 0. or not self.training:
-            return None
-        keep = 1.0 - self.drop_path_rate
-        N, H, W, _ = x.shape
-        mask = getattr(self, '_injected_drop_mask', None)
-        if mask is None:
-            mask = x.new_empty((N,)).bernoulli_(keep)
-            if keep > 0.0:
-                mask = mask / keep
-        return mask.to(x.device, torch.float32).repeat_interleave(H * W).contiguous()
-
     def forward(self, x, record=None):
         """x: NHWC.  Returns (x, loss or None)  (:387-396); both drop_path calls draw independent masks in the reference --
         an injected mask (tests) is shared by both, random masks are drawn twice."""
-        rs1 = self._row_scale(x)
+        rs1 = Fn.drop_path_row_scale(self, x)
         x = LF.AxpyFn.apply(self.attn(_bn(self.norm1, x)), x, self.layer_scale_1, rs1)
-        rs2 = self._row_scale(x)
+        rs2 = Fn.drop_path_row_scale(self, x)
         return self.mlp(_bn(self.norm2, x), self.layer_scale_2, x, rs2, record)
 
 

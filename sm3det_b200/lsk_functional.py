@@ -18,18 +18,11 @@ import torch.distributed as dist
 from torch.autograd import Function
 
 from . import ops
+from .functional import ROUTER_SAVED, _taps, _taps_flipped, route, router_backward, router_saved
 from .ops import EPI_GELU
 
 
 AMAX_RECORD = None   # parity tests set this to a list: LSKSelectFn appends the channel argmax [T] of every LSKblock (forward order)
-
-
-def _taps(w):              # [C,1,ks,ks] -> [ks*ks][C]
-    return w.reshape(w.shape[0], -1).t().contiguous()
-
-
-def _taps_flipped(w):
-    return w.flip(2, 3).reshape(w.shape[0], -1).t().contiguous()
 
 
 def _sync_active(sync):
@@ -328,9 +321,7 @@ class MoELinearFn(Function):
         ws, bs = experts[:E], experts[E:]
         Cout = ws[0].shape[0]
         train = any(ctx.needs_input_grad)
-        r = ops.moe_router(x2, wp, bp, sim, tau, T=T, Cc=Cin, E=E, k=k, w_noise=w_noise, noise=noise, save=train)
-        plan = ops.moe_plan(r['partials'], T=T, E=E, k=k)
-        slot_of, pair_token = ops.moe_assign(r['top_idx'], plan, T=T, E=E, k=k)
+        r, plan, slot_of, pair_token = route(x2, wp, bp, sim, tau, w_noise, noise, T=T, C=Cin, E=E, k=k, save=train)
         R = plan['max_rows']
         grouped = (plan['tile_group'], plan['num_m_tiles'])
         w0 = ws[0].view(Cout, Cin)
@@ -344,21 +335,21 @@ class MoELinearFn(Function):
             record.append(dict(x=x2, top_idx=r['top_idx'], top_gate=r['top_gate'], importance=plan['importance'],
                                load=plan['load'], loss=plan['loss'], y=y, counts=plan['counts']))
         if train:
-            ctx.noisy = noise is not None     # gates depend on w_noise whenever noise was added, also for k == E
-            ctx.save_for_backward(x2, o, wp, sim, tau, gamma, row_scale, r['top_idx'], r['top_gate'], r['logits'], r['p'],
-                                  slot_of, pair_token, plan['importance'], plan['seg_begin'], plan['seg_end'],
-                                  plan['tile_group'], plan['num_m_tiles'], w0, noise, r['sigma'], r['top_vals'],
-                                  r['top_idx_m'], plan['load'], w_noise)
+            ctx.save_for_backward(*router_saved(r, plan, sim, tau, noise, w_noise), x2, o, wp, gamma, row_scale, slot_of,
+                                  pair_token, plan['seg_begin'], plan['seg_end'], plan['tile_group'], plan['num_m_tiles'],
+                                  w0)
             ctx.E, ctx.k, ctx.R, ctx.lead = E, k, R, tuple(lead)
             ctx.wshape = tuple(ws[0].shape)
-            ctx.has_noise_param = w_noise is not None
             ctx.has_resid = resid is not None
         return out.view(*lead, Cout), plan['loss'].reshape(())
 
     @staticmethod
     def backward(ctx, dout, dloss):
-        (x2, o, wp, sim, tau, gamma, rs, top_idx, top_gate, logits, p, slot_of, pair_token, importance, seg_begin, seg_end,
-         tile_group, num_m_tiles, w0, noise, sigma, top_vals, top_idx_m, load, w_noise) = ctx.saved_tensors
+        saved = ctx.saved_tensors
+        router = saved[:ROUTER_SAVED]
+        (x2, o, wp, gamma, rs, slot_of, pair_token, seg_begin, seg_end, tile_group, num_m_tiles,
+         w0) = saved[ROUTER_SAVED:]
+        top_idx, top_gate = router[:2]
         E, k, R = ctx.E, ctx.k, ctx.R
         T, Cin = x2.shape
         Cout = w0.shape[0]
@@ -374,29 +365,8 @@ class MoELinearFn(Function):
         ops.colsum(d_o, dbs, rows=R, Cc=Cout, segs=segs, groups=E)
         dxp = torch.zeros((R, Cin), device=dev, dtype=torch.float32)
         ops.linear_dgrad(d_o, w0, out=dxp, grouped=grouped, w_group_stride=Cout * Cin)
-        P = wp.shape[0]
-        dtau = torch.zeros((1,), device=dev, dtype=torch.float32)
-        dsim = torch.zeros((P, E), device=dev, dtype=torch.float32)
-        lscale = dloss.reshape(1).contiguous().float()
-        noisy = dict(noise=noise, sigma=sigma, top_vals=top_vals, top_idx_m=top_idx_m, load=load) if ctx.noisy else None
-        dp, dr = ops.moe_router_bwd(p, sim, tau, top_idx, top_gate, dgate, logits, importance, lscale, dsim, dtau, T=T,
-                                    E=E, k=k, noisy=noisy)
-        dwp = torch.zeros_like(wp)
-        ops.linear_wgrad(dp, x2, dwp)
-        dbp = torch.zeros((P,), device=dev, dtype=torch.float32)
-        ops.colsum(dp, dbp, rows=T, Cc=P)
-        dx_r = ops.linear_dgrad(dp, wp)
-        dwn = None
-        if ctx.noisy:
-            wn_t = torch.zeros((32, Cin), device=dev, dtype=torch.float32)
-            wn_t[:E] = w_noise.t()
-            dwn_t = torch.zeros((32, Cin), device=dev, dtype=torch.float32)
-            ops.linear_wgrad(dr, x2, dwn_t)
-            dwn = dwn_t[:E].t().contiguous()
-            dx_r = ops.linear_dgrad(dr, wn_t, epilogue=ops.EPI_RESID, resid=dx_r)
+        dx_r, dwp, dbp, dsim, dtau, dwn = router_backward(router, x2, wp, dgate, dloss)
         dx = ops.gather_sum(dxp, slot_of, dx_r, T=T, Cc=Cin, k=k)
-        if dwn is None and ctx.has_noise_param:
-            dwn = torch.zeros((Cin, E), device=dev, dtype=torch.float32)
         dresid = dout if ctx.has_resid else None
         grads_e = [dws[e].view(ctx.wshape) for e in range(E)] + [dbs[e] for e in range(E)]
         return (dx.view(*ctx.lead, Cin), dwp, dbp, dsim, dtau, dwn, None, dgamma, dresid, None, None, None, None, *grads_e)
